@@ -7,6 +7,8 @@ import os
 
 import numpy as np
 
+from .opcodes import P_FIELD
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libaegolius_b200.so")
 
@@ -98,6 +100,10 @@ _SIGNATURES = {
                                 C.c_void_p, C.c_int, C.c_void_p]),
     "ab_edge_filter": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint32), C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "ab_signed_field": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint32), C.c_double, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
+    "ab_signed_mask": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint32), C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
+                                 C.c_void_p]),
+    "ab_signed_field_slab": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.c_uint32,
+                                       C.c_uint32, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "ab_vec_apply": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(ab_vec_op), C.c_uint32, C.c_int, C.c_int,
                                C.c_void_p]),
     "ab_vec_component": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_int, C.c_int, C.c_void_p, C.c_int,
@@ -155,8 +161,11 @@ class CProgram:
         n_blobs = len(self._blob_arrays)
         self._blobs = (ab_blob * max(1, n_blobs))()
         fields = {st["blob"] for st in getattr(prog, "stages", ())}  # P_FIELD inputs: device arrays, one value per point
+        read = {int(b) for c, b in zip(prog.ops["opcode"], prog.ops["b"]) if int(c) == P_FIELD}
         for i, b in enumerate(self._blob_arrays):
-            if i in fields:
+            if i in fields and i not in read and (device_blobs is None or device_blobs[i] is None):
+                self._blobs[i] = ab_blob(None, 0, 1, 1)  # a stage whose field this program never reads (pruned away)
+            elif i in fields:
                 if device_blobs is None or device_blobs[i] is None:
                     raise ValueError("this program has grid-stencil stages: evaluate it through aegolius_b200.create "
                                      "on a whole grid (the stages need the full field)")

@@ -1347,29 +1347,48 @@ extern "C" int ab_edge_filter(const void* field_dev, const uint32_t res[3], int 
 }
 
 // ---- signed: unsigned -> signed distance field (modifications.py:220-275) ---------------------------------------------------------
+static uint32_t mask_words(uint32_t n2) { return (n2 + 31u) / 32u; }
+
 template <typename T>
-static int signed_field_t(const void* field, const uint32_t res[3], double threshold, void* out, int device, cudaStream_t st) {
-  const uint64_t n = (uint64_t)res[0] * res[1] * res[2];
-  Field3 f{res[0], res[1], res[2]};
-  char* buf = nullptr;
+static int signed_mask_t(const void* field, const uint32_t res[3], double threshold, uint32_t* mask, int* flags, cudaStream_t st) {
+  const uint32_t words = mask_words(res[2]), wpb = std::min<uint32_t>(words, 8u);  // mask words (warps) per CTA
+  const dim3 g((words + wpb - 1) / wpb, res[1], res[0]);
+  ab_signed_mask_kernel<T><<<g, wpb * 32, 0, st>>>((const T*)field, Field3{res[0], res[1], res[2]}, words, (T)threshold, mask, flags);
+  CUDA_TRY(cudaGetLastError());
+  g_launches++;
+  return AB_OK;
+}
+
+// planes [x0, x1) of the signed field from the whole mask: the (2,2,1) smoothing reads interior planes i and i + 1, the face
+// clamp reads planes 1 and n0 - 2 instead of 0 and n0 - 1, so the interior is needed on [c(x0), c(x1 - 1) + 2) with
+// c = clamp to [1, n0 - 2]. The box filter runs on that block as if it were a whole field: at a cut its last plane is
+// reflected wrongly and never read; at the face n0 - 1 it reflects like the whole field (same taps, same order).
+template <typename T>
+static int signed_slab_t(const uint32_t* mask, const int* flags, const void* field, uint32_t field_plane0, const uint32_t res[3],
+                         uint32_t x0, uint32_t x1, void* out, int device, cudaStream_t st) {
+  const uint32_t n0 = res[0], n1 = res[1], n2 = res[2], words = mask_words(n2);
+  auto clampi = [&](uint32_t i) { return i < 1 ? 1u : (i > n0 - 2 ? n0 - 2 : i); };
+  const uint32_t s0 = clampi(x0), s1 = clampi(x1 - 1) + 2, m = s1 - s0;  // interior / smoothed planes [s0, s1)
+  const uint64_t nw = (uint64_t)m * n1 * words, ni = (uint64_t)m * n1 * n2, plane = (uint64_t)n1 * n2;
   auto al = [](uint64_t b) { return (b + 255) & ~255ull; };
-  const uint64_t off_par1 = al(n), off_int = off_par1 + al(n), off_smooth = off_int + al(n * sizeof(T)),
-                 off_flags = off_smooth + al(n * sizeof(T)), total = off_flags + 256;
+  const uint64_t off_int = 4 * al(nw * 4), off_smooth = off_int + al(ni * sizeof(T)), total = off_smooth + al(ni * sizeof(T));
+  char* buf = nullptr;
   CUDA_TRY(cudaMallocAsync((void**)&buf, total, st));
-  uint8_t *par0 = (uint8_t*)buf, *par1 = (uint8_t*)(buf + off_par1);
+  uint32_t* par = (uint32_t*)buf;
+  uint32_t *pin0 = par, *pout0 = (uint32_t*)(buf + al(nw * 4)), *pin1 = (uint32_t*)(buf + 2 * al(nw * 4)),
+           *pout1 = (uint32_t*)(buf + 3 * al(nw * 4));
   T *interior = (T*)(buf + off_int), *smooth = (T*)(buf + off_smooth);
-  int* flags = (int*)(buf + off_flags);
   int rc = AB_OK;
   do {
-    if (cudaMemsetAsync(flags, 0, 2 * sizeof(int), st) != cudaSuccess) { rc = fail(AB_ECUDA, "memset"); break; }
-    const uint64_t cols = (uint64_t)std::max(res[0], res[1]) * res[2];
-    ab_signed_scan_kernel<T><<<dim3((unsigned)((cols + 255) / 256), 2), 256, 0, st>>>((const T*)field, f, (T)threshold, par0, par1, flags);
-    const dim3 g3((res[2] + 255) / 256, res[1], res[0]);
-    ab_signed_interior_kernel<T><<<g3, 256, 0, st>>>(par0, par1, f, interior);
-    const uint32_t ks[3] = {2, 2, 1};
-    rc = box_filter_t<T>(interior, res, ks, 1, smooth, device, st);  // conv_averaging(interior, (2, 2, 1), 1)
+    const uint64_t cols = std::max<uint64_t>((uint64_t)n1 * words, (uint64_t)m * words);
+    ab_signed_scan_kernel<<<dim3((unsigned)((cols + 255) / 256), 2), 256, 0, st>>>(mask, n0, n1, words, s0, s1, pin0, pout0, pin1, pout1);
+    const Field3 fm{m, n1, n2};
+    ab_signed_interior_kernel<T><<<dim3((n2 + 255) / 256, n1, m), 256, 0, st>>>(pin0, pout0, pin1, pout1, fm, words, interior);
+    const uint32_t ks[3] = {2, 2, 1}, rm[3] = {m, n1, n2};
+    rc = box_filter_t<T>(interior, rm, ks, 1, smooth, device, st);  // conv_averaging(interior, (2, 2, 1), 1)
     if (rc) break;
-    ab_signed_apply_kernel<T><<<g3, 256, 0, st>>>((const T*)field, smooth, f, flags, (T*)out);
+    ab_signed_apply_kernel<T><<<dim3((n2 + 255) / 256, n1, x1 - x0), 256, 0, st>>>(
+        (const T*)field + (uint64_t)(x0 - field_plane0) * plane, smooth, Field3{n0, n1, n2}, x0, s0, flags, (T*)out);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { rc = fail(AB_ECUDA, "signed launch: %s", cudaGetErrorString(e)); break; }
     g_launches += 3;
@@ -1378,18 +1397,69 @@ static int signed_field_t(const void* field, const uint32_t res[3], double thres
   return rc;
 }
 
+static int check_signed_res(const uint32_t res[3]) {
+  if (res[0] < 3 || res[1] < 3 || res[2] < 3) return fail(AB_EINVAL, "signed needs at least 3 samples per axis (the reference pads an empty interior otherwise)");
+  if (res[0] > 65535 || res[1] > 65535) return fail(AB_ETOOLARGE, "field axis longer than 65535 samples");
+  return AB_OK;
+}
+
+extern "C" int ab_signed_mask(const void* field_dev, const uint32_t res[3], double threshold, int dtype, uint32_t* mask_dev,
+                              int* flags_dev, int device, void* stream) {
+  int rc = use_device(device);
+  if (rc) return rc;
+  rc = check_field_args(field_dev, res, mask_dev);
+  if (rc) return rc;
+  if (!flags_dev) return fail(AB_EINVAL, "null pointer");
+  if (res[0] > 65535 || res[1] > 65535) return fail(AB_ETOOLARGE, "field axis longer than 65535 samples");
+  if (dtype == AB_F32) return signed_mask_t<float>(field_dev, res, threshold, mask_dev, flags_dev, (cudaStream_t)stream);
+  if (dtype == AB_F64) return signed_mask_t<double>(field_dev, res, threshold, mask_dev, flags_dev, (cudaStream_t)stream);
+  return fail(AB_EINVAL, "bad dtype %d", dtype);
+}
+
+extern "C" int ab_signed_field_slab(const uint32_t* mask_dev, const int* flags_dev, const void* field_dev, uint32_t field_plane0,
+                                    const uint32_t res[3], uint32_t x0, uint32_t x1, int dtype, void* out_dev, int device,
+                                    void* stream) {
+  int rc = use_device(device);
+  if (rc) return rc;
+  rc = check_field_args(field_dev, res, out_dev);
+  if (rc) return rc;
+  if (!mask_dev || !flags_dev) return fail(AB_EINVAL, "null pointer");
+  rc = check_signed_res(res);
+  if (rc) return rc;
+  if (x0 >= x1 || x1 > res[0]) return fail(AB_EINVAL, "bad slab [%u, %u) of %u planes", x0, x1, res[0]);
+  if (field_plane0 > x0) return fail(AB_EINVAL, "field does not cover the slab");
+  if (field_dev == out_dev) return fail(AB_EINVAL, "signed cannot run in place");
+  if (dtype == AB_F32) return signed_slab_t<float>(mask_dev, flags_dev, field_dev, field_plane0, res, x0, x1, out_dev, device, (cudaStream_t)stream);
+  if (dtype == AB_F64) return signed_slab_t<double>(mask_dev, flags_dev, field_dev, field_plane0, res, x0, x1, out_dev, device, (cudaStream_t)stream);
+  return fail(AB_EINVAL, "bad dtype %d", dtype);
+}
+
 extern "C" int ab_signed_field(const void* field_dev, const uint32_t res[3], double threshold, int dtype, void* out_dev, int device,
                                void* stream) {
   int rc = use_device(device);
   if (rc) return rc;
   rc = check_field_args(field_dev, res, out_dev);
   if (rc) return rc;
-  if (res[0] < 3 || res[1] < 3 || res[2] < 3) return fail(AB_EINVAL, "signed needs at least 3 samples per axis (the reference pads an empty interior otherwise)");
-  if (res[0] > 65535 || res[1] > 65535) return fail(AB_ETOOLARGE, "field axis longer than 65535 samples");
+  rc = check_signed_res(res);
+  if (rc) return rc;
   if (field_dev == out_dev) return fail(AB_EINVAL, "signed cannot run in place");
-  if (dtype == AB_F32) return signed_field_t<float>(field_dev, res, threshold, out_dev, device, (cudaStream_t)stream);
-  if (dtype == AB_F64) return signed_field_t<double>(field_dev, res, threshold, out_dev, device, (cudaStream_t)stream);
-  return fail(AB_EINVAL, "bad dtype %d", dtype);
+  if (dtype != AB_F32 && dtype != AB_F64) return fail(AB_EINVAL, "bad dtype %d", dtype);
+  cudaStream_t st = (cudaStream_t)stream;
+  const uint64_t nw = (uint64_t)res[0] * res[1] * mask_words(res[2]);
+  char* buf = nullptr;
+  CUDA_TRY(cudaMallocAsync((void**)&buf, 256 + nw * 4, st));
+  int* flags = (int*)buf;
+  uint32_t* mask = (uint32_t*)(buf + 256);
+  do {
+    if (cudaMemsetAsync(flags, 0, 2 * sizeof(int), st) != cudaSuccess) { rc = fail(AB_ECUDA, "memset"); break; }
+    rc = dtype == AB_F32 ? signed_mask_t<float>(field_dev, res, threshold, mask, flags, st)
+                         : signed_mask_t<double>(field_dev, res, threshold, mask, flags, st);
+    if (rc) break;
+    rc = dtype == AB_F32 ? signed_slab_t<float>(mask, flags, field_dev, 0, res, 0, res[0], out_dev, device, st)
+                         : signed_slab_t<double>(mask, flags, field_dev, 0, res, 0, res[0], out_dev, device, st);
+  } while (0);
+  cudaFreeAsync(buf, st);
+  return rc;
 }
 
 static int check_vec_op(const ab_vec_op& op, uint32_t i, uint64_t n) {

@@ -194,74 +194,111 @@ __global__ void __launch_bounds__(256) ab_edge_kernel(const T* __restrict__ in, 
 // neighbour's value, and the field is negated where the result exceeds 1/2. If the field has a negative sample it is
 // returned untouched.
 //
-// ab_signed_scan_kernel: a thread owns one column along the scanned axis and marches it once, storing both prefix
-// parities per sample (bit 0: entries, bit 1: exits). blockIdx.y selects the axis: 0 scans along axis 0 (thread = (i1, i2)),
-// 1 scans along axis 1 (thread = (i0, i2)); threads are consecutive in i2, so every access is coalesced. It also raises
-// flags[0] when a sample is negative and flags[1] when one is NaN.
+// Along axis 0 a plane's interior depends on the whole column (the mirrored plane n0-1-i too), so the kernels work from a
+// packed boundary mask of the whole field: bit (i2 & 31) of word [i0][i1][i2 / 32] (rows padded to whole words), 1 bit per
+// sample. A slab of the field is signed from the whole mask plus its own planes of the field; the mask can be packed slab
+// by slab (by different ranks) and concatenated.
+
+// the mask of a C-ordered (n0, n1, n2) block of the field: one warp per mask word (__ballot_sync of 32 consecutive z);
+// flags[0] |= a sample is negative, flags[1] |= a sample is NaN
 template <typename T>
-__global__ void __launch_bounds__(256) ab_signed_scan_kernel(const T* __restrict__ field, Field3 f, T threshold, uint8_t* __restrict__ par0,
-                                                             uint8_t* __restrict__ par1, int* __restrict__ flags) {
-  const int axis = blockIdx.y;
-  const uint32_t ncols = (axis == 0 ? f.n1 : f.n0) * f.n2;
-  const uint32_t col = blockIdx.x * blockDim.x + threadIdx.x;
-  if (col >= ncols) return;
-  const uint32_t a = col / f.n2, i2 = col - a * f.n2;  // a = i1 (axis 0) or i0 (axis 1)
-  const uint64_t plane = (uint64_t)f.n1 * f.n2;
-  const uint64_t base = axis == 0 ? (uint64_t)a * f.n2 + i2 : (uint64_t)a * plane + i2;
-  const uint64_t step = axis == 0 ? plane : f.n2;
-  const uint32_t n = axis == 0 ? f.n0 : f.n1;
-  uint8_t* par = axis == 0 ? par0 : par1;
-  bool neg = false, nan = false;
-  unsigned p_in = 0, p_out = 0;
-  T cur = field[base];
-  bool b_prev = false, b_cur = cur < threshold;
-  for (uint32_t i = 0; i < n; i++) {
-    const T nxt = i + 1 < n ? field[base + (uint64_t)(i + 1) * step] : T(0);
-    const bool b_next = i + 1 < n ? nxt < threshold : false;
-    if (axis == 0) {
-      neg |= cur < T(0);
-      nan |= cur != cur;
-    }
-    if (i > 0 && b_cur && !b_prev) p_in ^= 1u;      // chu[i]  = boundary[i] & ~boundary[i-1]   (i >= 1)
-    if (i + 1 < n && b_cur && !b_next) p_out ^= 1u;  // chuu[i] = boundary[i] & ~boundary[i+1]   (i <= n-2)
-    par[base + (uint64_t)i * step] = (uint8_t)(p_in | (p_out << 1));
-    b_prev = b_cur;
-    b_cur = b_next;
-    cur = nxt;
+__global__ void __launch_bounds__(256) ab_signed_mask_kernel(const T* __restrict__ field, Field3 f, uint32_t words, T threshold,
+                                                             uint32_t* __restrict__ mask, int* __restrict__ flags) {
+  const uint32_t lane = threadIdx.x & 31u, w = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (w >= words) return;  // whole warps
+  const uint64_t row = (uint64_t)blockIdx.z * f.n1 + blockIdx.y;
+  const uint32_t i2 = w * 32u + lane;
+  bool b = false, neg = false, nan = false;
+  if (i2 < f.n2) {
+    const T v = field[row * f.n2 + i2];
+    b = v < threshold;
+    neg = v < T(0);
+    nan = v != v;
   }
-  if (neg) atomicOr(flags, 1);
-  if (nan) atomicOr(flags + 1, 1);
+  const unsigned word = __ballot_sync(0xffffffffu, b);
+  const bool any_neg = __any_sync(0xffffffffu, neg), any_nan = __any_sync(0xffffffffu, nan);
+  if (lane == 0) {
+    mask[row * words + w] = word;
+    if (any_neg) atomicOr(flags, 1);
+    if (any_nan) atomicOr(flags + 1, 1);
+  }
 }
 
-// interior = (in0[i0] | out0[n0-1-i0]) & (in1[i1] | out1[n1-1-i1]) as a 0 / 1 field of T
+// Bit-sliced crossing parities: a thread owns one mask word (32 columns) and marches it along the scanned axis, keeping
+// the entry and exit parities as words:  in ^= b & ~prev (entries counted from i = 1),  out ^= b & ~next (up to n-2).
+// It stores in(i) to pin[i] and out(i) to pout[n-1-i] for the positions i the caller asked for (plain stores, each slot
+// written once), so in | out at a position is the interior test along that axis.
+// blockIdx.y = 0: along axis 0, thread = (i1, word), stores planes [x0, x1) (slab-local);
+// blockIdx.y = 1: along axis 1 inside the planes [x0, x1), thread = (i0 - x0, word), stores every i1.
+__global__ void __launch_bounds__(256) ab_signed_scan_kernel(const uint32_t* __restrict__ mask, uint32_t n0, uint32_t n1,
+                                                             uint32_t words, uint32_t x0, uint32_t x1, uint32_t* __restrict__ pin0,
+                                                             uint32_t* __restrict__ pout0, uint32_t* __restrict__ pin1,
+                                                             uint32_t* __restrict__ pout1) {
+  const int axis = blockIdx.y;
+  const uint64_t plane_w = (uint64_t)n1 * words;
+  const uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  uint64_t src, step, dst, dstep;
+  uint32_t n, lo, hi;
+  uint32_t *pin, *pout;
+  if (axis == 0) {
+    if (c >= plane_w) return;
+    src = c; step = plane_w; n = n0; lo = x0; hi = x1; dst = c; dstep = plane_w; pin = pin0; pout = pout0;
+  } else {
+    if (c >= (uint64_t)(x1 - x0) * words) return;
+    const uint64_t p = c / words, w = c - p * words;
+    src = (x0 + p) * plane_w + w; step = words; n = n1; lo = 0; hi = n1; dst = p * plane_w + w; dstep = words;
+    pin = pin1; pout = pout1;
+  }
+  uint32_t in = 0, out = 0, prev = ~0u;
+  constexpr int U = 8;  // loads issued together: the march is latency-bound
+  for (uint32_t i0 = 0; i0 < n; i0 += U) {
+    uint32_t b[U + 1];
+#pragma unroll
+    for (int u = 0; u <= U; u++) b[u] = i0 + u < n ? mask[src + (uint64_t)(i0 + u) * step] : ~0u;  // ~0: no exit at n-1
+#pragma unroll
+    for (int u = 0; u < U; u++) {
+      const uint32_t i = i0 + u;
+      if (i >= n) break;
+      in ^= b[u] & ~prev;
+      out ^= b[u] & ~b[u + 1];
+      prev = b[u];
+      if (i >= lo && i < hi) pin[dst + (uint64_t)(i - lo) * dstep] = in;
+      const uint32_t j = n - 1 - i;
+      if (j >= lo && j < hi) pout[dst + (uint64_t)(j - lo) * dstep] = out;
+    }
+  }
+}
+
+// interior = (in0 | out0) & (in1 | out1) as a 0 / 1 field of T over the planes of the parity words
 template <typename T>
-__global__ void __launch_bounds__(256) ab_signed_interior_kernel(const uint8_t* __restrict__ par0, const uint8_t* __restrict__ par1, Field3 f,
-                                                                 T* __restrict__ interior) {
+__global__ void __launch_bounds__(256) ab_signed_interior_kernel(const uint32_t* __restrict__ pin0, const uint32_t* __restrict__ pout0,
+                                                                 const uint32_t* __restrict__ pin1, const uint32_t* __restrict__ pout1,
+                                                                 Field3 f, uint32_t words, T* __restrict__ interior) {
   const uint32_t i2 = blockIdx.x * blockDim.x + threadIdx.x, i1 = blockIdx.y, i0 = blockIdx.z;
   if (i2 >= f.n2) return;
-  const uint64_t plane = (uint64_t)f.n1 * f.n2;
-  const uint64_t k = i0 * plane + (uint64_t)i1 * f.n2 + i2;
-  const unsigned a = (par0[k] & 1u) | ((par0[(uint64_t)(f.n0 - 1 - i0) * plane + (uint64_t)i1 * f.n2 + i2] >> 1) & 1u);
-  const unsigned b = (par1[k] & 1u) | ((par1[i0 * plane + (uint64_t)(f.n1 - 1 - i1) * f.n2 + i2] >> 1) & 1u);
-  interior[k] = (a & b) ? T(1) : T(0);
+  const uint64_t kw = ((uint64_t)i0 * f.n1 + i1) * words + (i2 >> 5);
+  const uint32_t word = (pin0[kw] | pout0[kw]) & (pin1[kw] | pout1[kw]);
+  interior[((uint64_t)i0 * f.n1 + i1) * f.n2 + i2] = (word >> (i2 & 31u)) & 1u ? T(1) : T(0);
 }
 
-// out = field * (1 - 2 (smooth[clamped index] > 1/2)); untouched when the field had a negative sample (and no NaN: np.amin
-// of a field with a NaN is NaN, which is not < 0)
+// out = field * (1 - 2 (smooth[clamped index] > 1/2)) for the planes [x0, x0 + gridDim.z) of a field of f (global sizes);
+// `field` and `out` start at plane x0, `smooth` at plane s0. Untouched when the field had a negative sample (and no NaN:
+// np.amin of a field with a NaN is NaN, which is not < 0)
 template <typename T>
 __global__ void __launch_bounds__(256) ab_signed_apply_kernel(const T* __restrict__ field, const T* __restrict__ smooth, Field3 f,
-                                                              const int* __restrict__ flags, T* __restrict__ out) {
-  const uint32_t i2 = blockIdx.x * blockDim.x + threadIdx.x, i1 = blockIdx.y, i0 = blockIdx.z;
+                                                              uint32_t x0, uint32_t s0, const int* __restrict__ flags,
+                                                              T* __restrict__ out) {
+  const uint32_t i2 = blockIdx.x * blockDim.x + threadIdx.x, i1 = blockIdx.y, i0 = x0 + blockIdx.z;
   if (i2 >= f.n2) return;
   const uint64_t plane = (uint64_t)f.n1 * f.n2;
-  const uint64_t k = i0 * plane + (uint64_t)i1 * f.n2 + i2;
+  const uint64_t k = (uint64_t)blockIdx.z * plane + (uint64_t)i1 * f.n2 + i2;
   const T v = field[k];
   if (flags[0] && !flags[1]) {
     out[k] = v;
     return;
   }
   auto inner = [](uint32_t i, uint32_t n) { return i < 1 ? 1u : (i > n - 2 ? n - 2 : i); };  // [1:-1] then edge padding
-  const T s = smooth[inner(i0, f.n0) * plane + (uint64_t)inner(i1, f.n1) * f.n2 + inner(i2, f.n2)];
+  const T s = smooth[(uint64_t)(inner(i0, f.n0) - s0) * plane + (uint64_t)inner(i1, f.n1) * f.n2 + inner(i2, f.n2)];
   out[k] = s > T(0.5) ? -v : v;
 }
 

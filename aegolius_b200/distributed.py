@@ -106,14 +106,49 @@ def gather_rows(local_rows, spec, group=None):
     return out
 
 
+class _MaskLayout:
+    """The plane layout gather_field assembles: n0 planes of `per_plane` values."""
+
+    def __init__(self, n0, per_plane):
+        self.res = (n0, per_plane, 1)
+        self.n_points = n0 * per_plane
+
+
+class MaskGather:
+    """The boundary mask of a `signed` stage covers whole columns along x, so a rank cannot sign its slab from its own
+    planes alone. With this passed as engine.create_torch(mask_gather=), each rank packs the mask of its own slab
+    (`planes`, 1 bit per sample), the slabs are all-gathered in place (gather_field) and the negative / NaN flags are
+    max-reduced: 1/32 of a fp32 field crosses the ranks instead of every rank evaluating the whole grid."""
+
+    def __init__(self, spec, group=None):
+        world, rank = _world(group)
+        self.group = group
+        self.n0 = spec.res[0]
+        self.planes = rank_slab(self.n0, rank, world)
+
+    def __call__(self, local_words, words_per_plane, flags):
+        import torch.distributed as dist
+        dist.all_reduce(flags, op=dist.ReduceOp.MAX, group=self.group)
+        return gather_field(local_words, _MaskLayout(self.n0, words_per_plane), self.group)
+
+
+def _mask_gather(obj, spec, group):
+    from . import engine
+    world, _ = _world(group)
+    return MaskGather(spec, group) if world > 1 and engine._as_program(obj).stages else None
+
+
 def evaluate_sharded(obj, spec, *, dtype="f32", grad=None, group=None, gather=False):
     """Evaluates this rank's slab on its GPU (device = LOCAL_RANK). gather=True assembles the full field — and, with
-    grad=, the full (K, N) gradient — on every rank."""
+    grad=, the full (K, N) gradient — on every rank. Trees with grid-stencil stages recompute the halo their stencils need
+    on every rank (Program.stage_plan); their `signed` masks are all-gathered (MaskGather)."""
     from . import engine
     world, rank = _world(group)
     device = int(os.environ.get("LOCAL_RANK", "0"))
     slab = rank_slab(spec.res[0], rank, world)
-    res = engine.create_torch(obj, spec, dtype=dtype, grad=grad, device=device, slab=slab)
+    obj = engine._as_program(obj)
+    res = engine.create_torch(obj, spec, dtype=dtype, grad=grad, device=device, slab=slab,
+                              mask_gather=_mask_gather(obj, spec, group))
     if not gather or world == 1:
         return res
     if grad:
@@ -167,7 +202,8 @@ def from_sdf_sharded(obj, spec, *, dtype="f32", group=None, normalize=True, smoo
     x0, x1 = rank_slab(spec.res[0], rank, world)
     lo, hi = max(x0 - 1, 0), min(x1 + 1, spec.res[0])
     per_plane = spec.res[1] * spec.res[2]
-    halo = engine.create_torch(obj, spec, dtype=dtype, device=device, slab=(lo, hi))
+    obj = engine._as_program(obj)
+    halo = engine.create_torch(obj, spec, dtype=dtype, device=device, slab=(lo, hi), mask_gather=_mask_gather(obj, spec, group))
     res = spec.res if spec.res[2] > 1 or float(spec.size[2]) != 0.0 else spec.res[:2]
     vec = engine.from_sdf_torch(halo, res, slab=(x0, x1), field_plane0=lo, normalize=normalize, device=device)
     return halo[(x0 - lo) * per_plane:(x1 - lo) * per_plane], vec

@@ -207,6 +207,10 @@ class PinnedArray:
             pass
 
 
+_STAGED_ONLY = ("programs with grid stencils (conv_averaging / conv_edge_detection modifications) are evaluated on whole "
+                "grids only, without gradients")
+
+
 def create(obj, co, *, dtype="f32", grad=None, device=0, out=None, out_grad=None, slab=None):
     """Evaluates the SDF of `obj` on `co`.
 
@@ -223,13 +227,14 @@ def create(obj, co, *, dtype="f32", grad=None, device=0, out=None, out_grad=None
     gmode, rows = _grad_mode(grad)
     spec = detect_grid(co)
     if prog.stages:
-        if spec is None or slab is not None or rows:
-            raise NotImplementedError("programs with grid stencils (conv_averaging / conv_edge_detection modifications) are "
-                                      "evaluated on whole grids only, without gradients")
-        field = _create_staged(prog, spec, code, npdt, device)
-        if out is not None:
-            out[...] = field
-            return out
+        if spec is None or rows:
+            raise NotImplementedError(_STAGED_ONLY)
+        x0, x1 = (0, spec.res[0]) if slab is None else slab
+        n = (x1 - x0) * spec.res[1] * spec.res[2]
+        field = out if out is not None else np.empty(n, dtype=npdt)
+        if field.dtype != npdt or field.size != n or not field.flags.c_contiguous:
+            raise ValueError("out= must be a C-contiguous array of the evaluation dtype with N elements")
+        field[...] = _staged_torch(prog, spec, code, slab, None, device).cpu().numpy()
         return field
     _auto_specialize(prog, dtype, grad)
     if (spec is not None and not rows and out is None and prog.n_ops == 2
@@ -285,52 +290,96 @@ def grid_min_step(spec):
     return float(min(seps))
 
 
-def _create_staged(prog, spec, code, npdt, device):
-    """Programs with grid-stencil stages: for every stage, in program order, the prefix program ops[:k] is evaluated over the
-    whole grid on the device, filtered by ab_box_filter / ab_edge_filter, and bound to the P_FIELD op that replaced the
-    modification; the full program then runs once with all fields bound. Nothing but the result leaves the device."""
-    lib = cabi.lib()
-    n = spec.n_points
-    item = np.dtype(npdt).itemsize
-    g = cabi.make_grid(spec.size, spec.res)
-    res3 = (C.c_uint32 * 3)(*spec.res)
-    bound = [None] * len(prog.blobs)
-    bufs = []
+def _check_stage_grid(prog, spec):
+    for st in prog.stages:
+        want = tuple(resolution_conversion(int(r)) for r in st["res"] if r)
+        if want != tuple(spec.res[:len(want)]) or (len(want) == 2 and spec.res[2] != 1):
+            raise ValueError(f"Cannot reshape the pattern with shape ({spec.n_points},)")  # what smarter_reshape raises
+        if st["kind"] == 2 and min(spec.res) < 3:
+            raise ValueError("can't extend empty axis using modes other than 'constant' or 'empty'")  # np.pad
+
+
+def _staged_torch(prog, spec, code, slab, out, device, mask_gather=None):
+    """Programs with grid-stencil stages on the x-slab `slab` of a grid, into the torch tensor `out` (or a new one), on the
+    current torch stream. Program.stage_plan says on which planes each stage is needed: in program order, the pruned
+    prefix program ops[:k] is evaluated on the stage's planned range (with the fields of earlier stages bound), filtered by
+    ab_box_filter / ab_edge_filter as if that range were the whole field (reflection at a cut only corrupts the halo, which
+    the plan keeps out of the planes read later; at a grid face it reflects as the whole field does), or signed from the
+    boundary mask of the whole field (ab_signed_mask / ab_signed_field_slab); the result is bound to the P_FIELD op that
+    replaced the modification, slab-local, and the pruned program runs on the slab. Intermediate fields come from the torch
+    allocator; nothing is synchronised.
+
+    The mask of a signed stage covers every plane. Without `mask_gather` this process evaluates the stage's prefix on the
+    whole axis to pack it (the cost of one whole-grid prefix evaluation per signed stage, even for a thin slab). A sharded
+    evaluation passes a distributed.MaskGather: this process packs the mask of `mask_gather.planes` only, and
+    mask_gather(local_words, words_per_plane, flags) returns the whole mask (and max-reduces the two flags in place)."""
+    import torch
+    _check_stage_grid(prog, spec)
+    dev = torch.device("cuda", device)
+    stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+    tdt = torch.float32 if code == cabi.AB_F32 else torch.float64
     jdt = "f32" if code == cabi.AB_F32 else "f64"
-    try:
-        for st in sorted(prog.stages, key=prog.stage_op_index):
-            want = tuple(resolution_conversion(int(r)) for r in st["res"] if r)
-            if want != tuple(spec.res[:len(want)]) or (len(want) == 2 and spec.res[2] != 1):
-                raise ValueError(f"Cannot reshape the pattern with shape ({n},)")  # what smarter_reshape raises
-            pre = prog.prefix(prog.stage_op_index(st)).pruned()  # without the subtrees an earlier stage's field replaced
-            d_in, d_out = _DevBuf(n * item, device), _DevBuf(n * item, device)
-            bufs += [d_in, d_out]
-            cp = cabi.CProgram(pre, device_blobs=bound)
-            codegen.ensure(pre, jdt, None, is2d=_is_2d(spec))
-            cabi.check(lib.ab_eval_grid(cp.ref(), C.byref(g), code, cabi.AB_GRAD_NONE, d_in.ptr, None, 0, device, None))
-            if st["kind"] == 0:
-                ks = (C.c_uint32 * 3)(*st["ksize"])
-                cabi.check(lib.ab_box_filter(d_in.ptr, res3, ks, st["iterations"], code, d_out.ptr, device, None))
-            elif st["kind"] == 2:
-                if min(spec.res) < 3:
-                    raise ValueError("can't extend empty axis using modes other than 'constant' or 'empty'")  # np.pad
-                cabi.check(lib.ab_signed_field(d_in.ptr, res3, grid_min_step(spec), code, d_out.ptr, device, None))
-            else:
-                cabi.check(lib.ab_edge_filter(d_in.ptr, res3, code, d_out.ptr, device, None))
-            bound[st["blob"]] = (d_out.ptr.value, n)
-        d_res = _DevBuf(n * item, device)
-        bufs.append(d_res)
-        final = prog.pruned()  # the subtrees that fed the stages are dead code now: P_FIELD overwrites their value
-        cp = cabi.CProgram(final, device_blobs=bound)
-        codegen.ensure(final, jdt, None, is2d=_is_2d(spec))
-        cabi.check(lib.ab_eval_grid(cp.ref(), C.byref(g), code, cabi.AB_GRAD_NONE, d_res.ptr, None, 0, device, None))
-        field = np.empty(n, dtype=npdt)
-        d_res.download(field)
-        cabi.check(lib.ab_stream_sync(device, None))
-    finally:
-        for b in bufs:
-            b.close()
-    return field
+    item = 4 if code == cabi.AB_F32 else 8
+    lib = cabi.lib()
+    n0, pp = spec.res[0], spec.res[1] * spec.res[2]
+    x0, x1 = (0, n0) if slab is None else (int(slab[0]), int(slab[1]))
+    plan, _ = prog.stage_plan(spec.res, (x0, x1), None if mask_gather is None else mask_gather.planes)
+    fields = {}  # blob -> (device tensor, its first plane)
+    res3 = lambda m: (C.c_uint32 * 3)(m, spec.res[1], spec.res[2])
+
+    def run(p, lo, hi, dst):
+        bound = [None] * len(prog.blobs)
+        for blob, (t, p0) in fields.items():
+            if p0 <= lo and hi - p0 <= t.numel() // pp:  # the plan makes every field a program reads cover its range
+                bound[blob] = (t.data_ptr() + (lo - p0) * pp * item, (hi - lo) * pp)
+        cp = cabi.CProgram(p, device_blobs=bound)
+        codegen.ensure(p, jdt, None, is2d=_is_2d(spec))
+        g = cabi.make_grid(spec.size, spec.res, (lo, hi))
+        cabi.check(lib.ab_eval_grid(cp.ref(), C.byref(g), code, cabi.AB_GRAD_NONE, C.c_void_p(dst.data_ptr()), None, 0,
+                                    device, stream))
+
+    for st, ev, valid in plan:
+        if ev is None:
+            continue  # no later program reads this stage
+        lo, hi = ev
+        pre = prog.prefix(prog.stage_op_index(st)).pruned()  # without the subtrees an earlier stage's field replaced
+        src = torch.empty((hi - lo) * pp, dtype=tdt, device=dev)
+        run(pre, lo, hi, src)
+        if st["kind"] == 0:
+            dst = torch.empty_like(src)
+            ks = (C.c_uint32 * 3)(*st["ksize"])
+            cabi.check(lib.ab_box_filter(C.c_void_p(src.data_ptr()), res3(hi - lo), ks, st["iterations"], code,
+                                         C.c_void_p(dst.data_ptr()), device, stream))
+            fields[st["blob"]] = (dst, lo)
+        elif st["kind"] == 1:
+            dst = torch.empty_like(src)
+            cabi.check(lib.ab_edge_filter(C.c_void_p(src.data_ptr()), res3(hi - lo), code, C.c_void_p(dst.data_ptr()),
+                                          device, stream))
+            fields[st["blob"]] = (dst, lo)
+        else:
+            words = (spec.res[2] + 31) // 32
+            wpp = spec.res[1] * words  # mask words per plane
+            flags = torch.zeros(2, dtype=torch.int32, device=dev)
+            m0, m1 = (0, n0) if mask_gather is None else mask_gather.planes
+            mask = torch.empty((m1 - m0) * wpp, dtype=torch.int32, device=dev)
+            cabi.check(lib.ab_signed_mask(C.c_void_p(src.data_ptr() + (m0 - lo) * pp * item), res3(m1 - m0),
+                                          grid_min_step(spec), code, C.c_void_p(mask.data_ptr()),
+                                          C.c_void_p(flags.data_ptr()), device, stream))
+            if mask_gather is not None:
+                mask = mask_gather(mask, wpp, flags)
+            dst = torch.empty((valid[1] - valid[0]) * pp, dtype=tdt, device=dev)
+            cabi.check(lib.ab_signed_field_slab(C.c_void_p(mask.data_ptr()), C.c_void_p(flags.data_ptr()),
+                                                C.c_void_p(src.data_ptr()), lo, (C.c_uint32 * 3)(*spec.res), valid[0],
+                                                valid[1], code, C.c_void_p(dst.data_ptr()), device, stream))
+            fields[st["blob"]] = (dst, valid[0])
+        del src
+    n = (x1 - x0) * pp
+    if out is None:
+        out = torch.empty(n, dtype=tdt, device=dev)
+    elif out.numel() != n or out.dtype != tdt or not out.is_contiguous() or out.device != dev:
+        raise ValueError("out= must be a contiguous CUDA tensor of the evaluation dtype with one value per slab sample")
+    run(prog.pruned(), x0, x1, out)  # the subtrees that fed the stages are dead code now: P_FIELD overwrites their value
+    return out
 
 
 def create_with_gradient(obj, co, **kw):
@@ -449,13 +498,19 @@ def value_and_grad(geometry, spec, target, *, dtype="f32", device=0, post=None, 
 # ---- device-resident evaluation (torch owns the memory and the stream) ------------------------------------------------------
 
 
-def create_torch(obj, spec: GridSpec, *, dtype="f32", grad=None, device=0, slab=None, out=None, out_grad=None):
+def create_torch(obj, spec: GridSpec, *, dtype="f32", grad=None, device=0, slab=None, out=None, out_grad=None,
+                 mask_gather=None):
     """Grid evaluation into torch CUDA tensors on the current torch stream (no host copy). Returns field
-    (and gradient (3,N) view of a row-padded buffer)."""
+    (and gradient (3,N) view of a row-padded buffer). Programs with grid-stencil stages evaluate their stages on the
+    slab plus the halo they need (_staged_torch, where `mask_gather` is described); they take no gradient."""
     import torch
     prog = _as_program(obj)
-    _auto_specialize(prog, dtype, grad)
     code, npdt = _dtype(dtype)
+    if prog.stages:
+        if grad not in (None, False, "none"):
+            raise NotImplementedError(_STAGED_ONLY)
+        return _staged_torch(prog, spec, code, slab, out, device, mask_gather)
+    _auto_specialize(prog, dtype, grad)
     codegen.ensure(prog, "f32" if code == cabi.AB_F32 else "f64", grad, is2d=_is_2d(spec))
     tdt = torch.float32 if code == cabi.AB_F32 else torch.float64
     gmode, rows = _grad_mode(grad)

@@ -354,7 +354,7 @@ class ModifyObject:
 
     def signed(self, co_resolution):
         """modifications.py:220-275: unsigned -> signed distance field on a 3D grid (a whole-grid post-pass, like the
-        convolution modifications: flattened into a stencil stage, engine._create_staged)."""
+        convolution modifications: flattened into a stencil stage, engine._staged_torch)."""
         return self._add("signed", co_resolution=co_resolution)
 
     # grid stencils (modifications.py:1586-1637): evaluated by separate kernels between two interpreter launches

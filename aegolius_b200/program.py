@@ -33,7 +33,7 @@ class Program:
         self.n_vslots = int(n_vslots)
         self.dargs = None
         # grid-stencil stages (conv_averaging / conv_edge_detection used as modifications): each entry names the P_FIELD
-        # blob it feeds and the stencil to run on the field accumulated by ops[:op_index] (see engine._create_staged)
+        # blob it feeds and the stencil to run on the field accumulated by ops[:op_index] (see engine._staged_torch)
         self.stages = [dict(st) for st in stages]
 
     @property
@@ -79,6 +79,57 @@ class Program:
         pre = Program(ops, self.args, self.blobs, self.n_pslots, self.n_vslots,
                       [st for st in self.stages if self.stage_op_index(st) < op_index])
         return pre
+
+    def stage_plan(self, res, slab=None, mask_planes=None):
+        """Which planes each stencil stage must be computed on so that the program is exact on the x-slab `slab` of a grid
+        of `res` samples (default: the whole grid). Returns (stages, final): for each stage in program order a tuple
+        (stage, eval, valid), where `eval` is the plane range on which its pruned prefix program is evaluated and `valid`
+        the range on which its filtered field must be exact (both None when no later program reads the stage), and `final`
+        the slab itself. Ranges are half-open (lo, hi) and lie in [0, res[0]).
+
+        The halo along x, per stage: a box filter of axis-0 size k and `it` iterations reads it * ((k - 1) // 2) planes
+        below and it * (k // 2) above (the even-kernel tap placement of ab_box_filter); when k exceeds the axis, reflection
+        can wrap past both faces, and the whole axis is used. The edge filter reads one plane on each side (x is a
+        stencil axis in 2D and 3D). `signed` reads its field only on its own planes, but its boundary mask covers whole
+        columns: its prefix is also evaluated on `mask_planes`, the planes whose mask this process packs itself (default:
+        all; a sharded evaluation packs its own slab and all-gathers the rest). A stage's field must be exact on the union
+        of the eval ranges of every later program whose pruned form still reads it."""
+        n0 = int(res[0])
+        x0, x1 = (0, n0) if slab is None else (int(slab[0]), int(slab[1]))
+        if not 0 <= x0 < x1 <= n0:
+            raise ValueError(f"slab ({x0}, {x1}) is not a non-empty plane range of [0, {n0})")
+        m0, m1 = (0, n0) if mask_planes is None else (int(mask_planes[0]), int(mask_planes[1]))
+        order = sorted(self.stages, key=self.stage_op_index)
+        need = [None] * len(order)
+
+        def widen(i, rng):
+            need[i] = rng if need[i] is None else (min(need[i][0], rng[0]), max(need[i][1], rng[1]))
+
+        def reads(prog, rng):
+            live = {int(b) for c, b in zip(prog.ops["opcode"], prog.ops["b"]) if int(c) == oc.P_FIELD}
+            for i, st in enumerate(order):
+                if st["blob"] in live:
+                    widen(i, rng)
+
+        reads(self.pruned(), (x0, x1))
+        plan = [None] * len(order)
+        for i in range(len(order) - 1, -1, -1):
+            st, valid = order[i], need[i]
+            if valid is None:
+                plan[i] = (st, None, None)
+                continue
+            lo, hi = valid
+            if st["kind"] == 0:
+                k, it = int(st["ksize"][0]), int(st["iterations"])
+                lo, hi = (0, n0) if k > n0 else (lo - it * ((k - 1) // 2), hi + it * (k // 2))
+            elif st["kind"] == 1:
+                lo, hi = lo - 1, hi + 1
+            else:
+                lo, hi = min(lo, m0), max(hi, m1)
+            ev = (max(lo, 0), min(hi, n0))
+            plan[i] = (st, ev, valid)
+            reads(self.prefix(self.stage_op_index(st)).pruned(), ev)
+        return plan, (x0, x1)
 
     def pruned(self):
         """Dead-code elimination by one backward liveness pass over the op list (registers: the point p, the value acc,
@@ -534,7 +585,7 @@ class _Builder:
             self.stages.append(dict(blob=b, kind=2, ksize=(2, 2, 1), iterations=1, res=res))
             post.append((oc.P_FIELD, b, []))
         elif name in ("conv_averaging", "conv_edge_detection"):
-            # grid stencils (modifications.py:1586-1637): the field accumulated so far is filtered over the whole grid by
+            # grid stencils (modifications.py:1586-1637): the field accumulated so far is filtered on the grid by
             # a separate kernel and comes back through a P_FIELD op; engine.create runs the stages in order
             res = tuple(int(r) for r in np.asarray(p["co_resolution"]).reshape(-1))
             if len(res) not in (2, 3):

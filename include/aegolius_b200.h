@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define AB_VERSION 100 /* 0.1.0 */
+#define AB_VERSION 101 /* 0.1.1 */
 
 typedef enum ab_status {
   AB_OK = 0,
@@ -274,6 +274,18 @@ int ab_edge_filter(const void* field_dev, const uint32_t res[3], int dtype, void
  * copied through (:234-235). Every axis needs >= 3 samples. Asynchronous on `stream`; out_dev != field_dev. */
 int ab_signed_field(const void* field_dev, const uint32_t res[3], double threshold, int dtype, void* out_dev, int device,
                     void* stream);
+/* The same, a slab at a time. ab_signed_mask packs the boundary mask (field < threshold) of a C-ordered block of res[3]
+ * samples (planes of the field): bit (i2 % 32) of uint32 word [i0][i1][i2 / 32], rows padded to whole words, so the
+ * masks of consecutive slabs concatenate into the mask of the field. It ORs 1 into flags_dev[0] when a sample is negative
+ * and into flags_dev[1] when one is NaN (the caller zeroes the two ints). */
+int ab_signed_mask(const void* field_dev, const uint32_t res[3], double threshold, int dtype, uint32_t* mask_dev,
+                   int* flags_dev, int device, void* stream);
+/* Planes [x0, x1) of the signed field of a field of res[3] samples, from the mask and flags of the WHOLE field and the
+ * field's own values: field_dev holds planes [field_plane0, ...) (field_plane0 <= x0), out_dev receives planes [x0, x1).
+ * The planes concatenate bit-identically to ab_signed_field. Every axis needs >= 3 samples. */
+int ab_signed_field_slab(const uint32_t* mask_dev, const int* flags_dev, const void* field_dev, uint32_t field_plane0,
+                         const uint32_t res[3], uint32_t x0, uint32_t x1, int dtype, void* out_dev, int device,
+                         void* stream);
 
 /* Vector-field modifiers (vector_modification_functions.py:14-172; methods modifications.py:1712-1971). */
 #define AB_MAX_VEC_OPS 32
