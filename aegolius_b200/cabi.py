@@ -28,7 +28,7 @@ class ab_blob(C.Structure):
 class ab_program(C.Structure):
     _fields_ = [("ops", C.c_void_p), ("n_ops", C.c_uint32), ("args", C.c_void_p), ("n_args", C.c_uint32),
                 ("dargs", C.c_void_p), ("blobs", C.POINTER(ab_blob)), ("n_blobs", C.c_uint32),
-                ("n_pslots", C.c_uint32), ("n_vslots", C.c_uint32)]
+                ("n_pslots", C.c_uint32), ("n_vslots", C.c_uint32), ("dblobs", C.POINTER(ab_blob))]
 
 
 class ab_grid(C.Structure):
@@ -104,6 +104,9 @@ _SIGNATURES = {
                                  C.c_void_p]),
     "ab_signed_field_slab": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.c_uint32,
                                        C.c_uint32, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
+    "ab_signed_field_slab_tangent": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
+                                               C.POINTER(C.c_uint32), C.c_uint32, C.c_uint32, C.c_int, C.c_void_p,
+                                               C.c_void_p, C.c_int, C.c_void_p]),
     "ab_vec_apply": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(ab_vec_op), C.c_uint32, C.c_int, C.c_int,
                                C.c_void_p]),
     "ab_vec_component": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_int, C.c_int, C.c_void_p, C.c_int,
@@ -152,9 +155,10 @@ def launch_count() -> int:
 
 
 class CProgram:
-    """Keeps the numpy buffers of a Program alive and exposes an ab_program struct."""
+    """Keeps the numpy buffers of a Program alive and exposes an ab_program struct. `device_blobs[b]` = (pointer, count) binds
+    the device field of a P_FIELD blob; `device_dblobs[b]` = (pointer, count) its tangent row (AB_GRAD_PARAM)."""
 
-    def __init__(self, prog, device_blobs=None):
+    def __init__(self, prog, device_blobs=None, device_dblobs=None):
         self._ops = np.ascontiguousarray(prog.ops)
         self._args = np.ascontiguousarray(prog.args, dtype=np.float64)
         self._blob_arrays = [np.ascontiguousarray(b, dtype=np.float64) for b in prog.blobs]
@@ -180,9 +184,15 @@ class CProgram:
             self._dargs = np.ascontiguousarray(prog.dargs, dtype=np.float64)
             if self._dargs.shape != self._args.shape:
                 raise ValueError("Program.dargs must have the shape of Program.args")
+        self._dblobs = None
+        if device_dblobs is not None:
+            self._dblobs = (ab_blob * max(1, n_blobs))()
+            for i, d in enumerate(device_dblobs):
+                if d is not None:
+                    self._dblobs[i] = ab_blob(d[0], d[1], 1, 1)
         self.struct = ab_program(self._ops.ctypes.data, self._ops.shape[0], self._args.ctypes.data,
                                  self._args.shape[0], self._dargs.ctypes.data if self._dargs is not None else None,
-                                 self._blobs, n_blobs, prog.n_pslots, prog.n_vslots)
+                                 self._blobs, n_blobs, prog.n_pslots, prog.n_vslots, self._dblobs)
 
     def ref(self):
         return C.byref(self.struct)

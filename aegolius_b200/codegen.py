@@ -265,7 +265,10 @@ class _Emitter:
         elif code == oc.P_AXIS:
             e(f"    {{ auto a = {A}; acc = {self.leaf_point}.{xyz[a]} - a[0]; }}")
         elif code == oc.P_FIELD:
-            e(f"    load_field(kp.blob[{b}], idx, kp.n, acc);")
+            if self.param:  # the stencil's tangent row rides along (ab_program.dblobs)
+                e(f"    load_field(kp.blob[{b}], kp.dblob[{b}], idx, kp.n, acc);")
+            else:
+                e(f"    load_field(kp.blob[{b}], idx, kp.n, acc);")
         elif code == oc.P_POINT_CLOUD:
             e(f"    acc = prim_point_cloud<S, T>({self.leaf_point}, kp.blob[{b}], kp.blob_count[{b}], {a}, kp.blob_tree[{b}]);")
         else:

@@ -589,11 +589,13 @@ static int run_program(const ab_program* prog, const EvalTarget<T>& tg, int grad
 
   std::vector<void*> temp_blobs;
   const char* field_base[AB_MAX_BLOBS] = {nullptr, nullptr, nullptr, nullptr};
+  const char* dfield_base[AB_MAX_BLOBS] = {nullptr, nullptr, nullptr, nullptr};
   static_assert(AB_MAX_BLOBS == 4, "field_base initialiser");
   for (uint32_t b = 0; b < AB_MAX_BLOBS; b++) {
     kp.blob[b] = nullptr;
     kp.blob_count[b] = 0;
     kp.blob_tree[b] = nullptr;
+    kp.dblob[b] = nullptr;
   }
   bool blob_used[AB_MAX_BLOBS] = {false, false, false, false};
   for (uint32_t i = 0; i < prog->n_ops; i++)
@@ -603,10 +605,18 @@ static int run_program(const ab_program* prog, const EvalTarget<T>& tg, int grad
     if (!blob_used[b]) continue;  // e.g. the not-yet-computed field of a later stencil stage in a prefix program
     if (bl.dim == 1) {  // a per-point field (P_FIELD): used in place, advanced with the output pointer per launch
       if (!bl.data || !bl.on_device || bl.count < tg.n) return fail(AB_EINVAL, "field blob %u must be a device array of >= %llu values", b, (unsigned long long)tg.n);
-      if (grad_mode != AB_GRAD_NONE) return fail(AB_EUNSUPPORTED_OP, "no derivative passes through a grid stencil (P_FIELD, blob %u)", b);
+      if (grad_mode == AB_GRAD_SPATIAL) return fail(AB_EUNSUPPORTED_OP, "no derivative passes through a grid stencil (P_FIELD, blob %u)", b);
       field_base[b] = (const char*)bl.data;
       kp.blob[b] = bl.data;
       kp.blob_count[b] = 0;
+      if (grad_mode == AB_GRAD_PARAM) {  // the stencil's tangent row, bound and advanced like the field
+        const ab_blob* db = prog->dblobs ? &prog->dblobs[b] : nullptr;
+        if (!db || !db->data || !db->on_device || db->dim != 1 || db->count < tg.n)
+          return fail(AB_EINVAL, "AB_GRAD_PARAM: field blob %u needs a device tangent row (ab_program.dblobs) of >= %llu values", b,
+                      (unsigned long long)tg.n);
+        dfield_base[b] = (const char*)db->data;
+        kp.dblob[b] = db->data;
+      }
       continue;
     }
     if (!bl.data || bl.count == 0 || bl.count > 0xffffffffull) return fail(AB_EINVAL, "blob %u empty or too large", b);
@@ -675,7 +685,10 @@ static int run_program(const ab_program* prog, const EvalTarget<T>& tg, int grad
     kp.target = tg.target ? tg.target + done : nullptr;
     kp.loss_accum = tg.loss_accum;
     for (uint32_t b = 0; b < AB_MAX_BLOBS; b++)
-      if (field_base[b]) kp.blob[b] = field_base[b] + done * sizeof(T);
+      if (field_base[b]) {
+        kp.blob[b] = field_base[b] + done * sizeof(T);
+        if (dfield_base[b]) kp.dblob[b] = dfield_base[b] + done * sizeof(T);
+      }
     if (tg.grid_mode) {
       if (tg.g.is2d) kp.g.i1_begin = tg.g.i1_begin + (uint32_t)(done / tg.g.n2);
       else kp.g.i0_begin = tg.g.i0_begin + (uint32_t)(done / tg.g.plane);
@@ -1364,8 +1377,9 @@ static int signed_mask_t(const void* field, const uint32_t res[3], double thresh
 // c = clamp to [1, n0 - 2]. The box filter runs on that block as if it were a whole field: at a cut its last plane is
 // reflected wrongly and never read; at the face n0 - 1 it reflects like the whole field (same taps, same order).
 template <typename T>
-static int signed_slab_t(const uint32_t* mask, const int* flags, const void* field, uint32_t field_plane0, const uint32_t res[3],
-                         uint32_t x0, uint32_t x1, void* out, int device, cudaStream_t st) {
+static int signed_slab_t(const uint32_t* mask, const int* flags, const void* field, const void* tangent, uint32_t field_plane0,
+                         const uint32_t res[3], uint32_t x0, uint32_t x1, void* out, void* out_tangent, int device,
+                         cudaStream_t st) {
   const uint32_t n0 = res[0], n1 = res[1], n2 = res[2], words = mask_words(n2);
   auto clampi = [&](uint32_t i) { return i < 1 ? 1u : (i > n0 - 2 ? n0 - 2 : i); };
   const uint32_t s0 = clampi(x0), s1 = clampi(x1 - 1) + 2, m = s1 - s0;  // interior / smoothed planes [s0, s1)
@@ -1387,8 +1401,14 @@ static int signed_slab_t(const uint32_t* mask, const int* flags, const void* fie
     const uint32_t ks[3] = {2, 2, 1}, rm[3] = {m, n1, n2};
     rc = box_filter_t<T>(interior, rm, ks, 1, smooth, device, st);  // conv_averaging(interior, (2, 2, 1), 1)
     if (rc) break;
-    ab_signed_apply_kernel<T><<<dim3((n2 + 255) / 256, n1, x1 - x0), 256, 0, st>>>(
-        (const T*)field + (uint64_t)(x0 - field_plane0) * plane, smooth, Field3{n0, n1, n2}, x0, s0, flags, (T*)out);
+    const dim3 ga((n2 + 255) / 256, n1, x1 - x0);
+    const uint64_t skip = (uint64_t)(x0 - field_plane0) * plane;
+    if (tangent)  // the same sign per sample on the tangent row (tangent pointers null: value only)
+      ab_signed_apply_kernel<T, true><<<ga, 256, 0, st>>>((const T*)field + skip, (const T*)tangent + skip, smooth,
+                                                          Field3{n0, n1, n2}, x0, s0, flags, (T*)out, (T*)out_tangent);
+    else
+      ab_signed_apply_kernel<T, false><<<ga, 256, 0, st>>>((const T*)field + skip, nullptr, smooth, Field3{n0, n1, n2}, x0, s0,
+                                                           flags, (T*)out, nullptr);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { rc = fail(AB_ECUDA, "signed launch: %s", cudaGetErrorString(e)); break; }
     g_launches += 3;
@@ -1429,8 +1449,29 @@ extern "C" int ab_signed_field_slab(const uint32_t* mask_dev, const int* flags_d
   if (x0 >= x1 || x1 > res[0]) return fail(AB_EINVAL, "bad slab [%u, %u) of %u planes", x0, x1, res[0]);
   if (field_plane0 > x0) return fail(AB_EINVAL, "field does not cover the slab");
   if (field_dev == out_dev) return fail(AB_EINVAL, "signed cannot run in place");
-  if (dtype == AB_F32) return signed_slab_t<float>(mask_dev, flags_dev, field_dev, field_plane0, res, x0, x1, out_dev, device, (cudaStream_t)stream);
-  if (dtype == AB_F64) return signed_slab_t<double>(mask_dev, flags_dev, field_dev, field_plane0, res, x0, x1, out_dev, device, (cudaStream_t)stream);
+  if (dtype == AB_F32) return signed_slab_t<float>(mask_dev, flags_dev, field_dev, nullptr, field_plane0, res, x0, x1, out_dev, nullptr, device, (cudaStream_t)stream);
+  if (dtype == AB_F64) return signed_slab_t<double>(mask_dev, flags_dev, field_dev, nullptr, field_plane0, res, x0, x1, out_dev, nullptr, device, (cudaStream_t)stream);
+  return fail(AB_EINVAL, "bad dtype %d", dtype);
+}
+
+extern "C" int ab_signed_field_slab_tangent(const uint32_t* mask_dev, const int* flags_dev, const void* field_dev,
+                                            const void* tangent_dev, uint32_t field_plane0, const uint32_t res[3], uint32_t x0,
+                                            uint32_t x1, int dtype, void* out_dev, void* out_tangent_dev, int device,
+                                            void* stream) {
+  int rc = use_device(device);
+  if (rc) return rc;
+  rc = check_field_args(field_dev, res, out_dev);
+  if (rc) return rc;
+  if (!mask_dev || !flags_dev || !tangent_dev || !out_tangent_dev) return fail(AB_EINVAL, "null pointer");
+  rc = check_signed_res(res);
+  if (rc) return rc;
+  if (x0 >= x1 || x1 > res[0]) return fail(AB_EINVAL, "bad slab [%u, %u) of %u planes", x0, x1, res[0]);
+  if (field_plane0 > x0) return fail(AB_EINVAL, "field does not cover the slab");
+  if (field_dev == out_dev || tangent_dev == out_tangent_dev || field_dev == out_tangent_dev || tangent_dev == out_dev ||
+      out_dev == out_tangent_dev)
+    return fail(AB_EINVAL, "signed cannot run in place (inputs, outputs: four distinct buffers)");
+  if (dtype == AB_F32) return signed_slab_t<float>(mask_dev, flags_dev, field_dev, tangent_dev, field_plane0, res, x0, x1, out_dev, out_tangent_dev, device, (cudaStream_t)stream);
+  if (dtype == AB_F64) return signed_slab_t<double>(mask_dev, flags_dev, field_dev, tangent_dev, field_plane0, res, x0, x1, out_dev, out_tangent_dev, device, (cudaStream_t)stream);
   return fail(AB_EINVAL, "bad dtype %d", dtype);
 }
 
@@ -1455,8 +1496,8 @@ extern "C" int ab_signed_field(const void* field_dev, const uint32_t res[3], dou
     rc = dtype == AB_F32 ? signed_mask_t<float>(field_dev, res, threshold, mask, flags, st)
                          : signed_mask_t<double>(field_dev, res, threshold, mask, flags, st);
     if (rc) break;
-    rc = dtype == AB_F32 ? signed_slab_t<float>(mask, flags, field_dev, 0, res, 0, res[0], out_dev, device, st)
-                         : signed_slab_t<double>(mask, flags, field_dev, 0, res, 0, res[0], out_dev, device, st);
+    rc = dtype == AB_F32 ? signed_slab_t<float>(mask, flags, field_dev, nullptr, 0, res, 0, res[0], out_dev, nullptr, device, st)
+                         : signed_slab_t<double>(mask, flags, field_dev, nullptr, 0, res, 0, res[0], out_dev, nullptr, device, st);
   } while (0);
   cudaFreeAsync(buf, st);
   return rc;

@@ -283,11 +283,13 @@ __global__ void __launch_bounds__(256) ab_signed_interior_kernel(const uint32_t*
 
 // out = field * (1 - 2 (smooth[clamped index] > 1/2)) for the planes [x0, x0 + gridDim.z) of a field of f (global sizes);
 // `field` and `out` start at plane x0, `smooth` at plane s0. Untouched when the field had a negative sample (and no NaN:
-// np.amin of a field with a NaN is NaN, which is not < 0)
-template <typename T>
-__global__ void __launch_bounds__(256) ab_signed_apply_kernel(const T* __restrict__ field, const T* __restrict__ smooth, Field3 f,
-                                                              uint32_t x0, uint32_t s0, const int* __restrict__ flags,
-                                                              T* __restrict__ out) {
+// np.amin of a field with a NaN is NaN, which is not < 0). TANGENT: the same sign applied to `tangent` -> `out_tangent`
+// (laid out like field / out): the sign pattern is piecewise constant in the parameter, so it is the derivative
+template <typename T, bool TANGENT>
+__global__ void __launch_bounds__(256) ab_signed_apply_kernel(const T* __restrict__ field, const T* __restrict__ tangent,
+                                                              const T* __restrict__ smooth, Field3 f, uint32_t x0, uint32_t s0,
+                                                              const int* __restrict__ flags, T* __restrict__ out,
+                                                              T* __restrict__ out_tangent) {
   const uint32_t i2 = blockIdx.x * blockDim.x + threadIdx.x, i1 = blockIdx.y, i0 = x0 + blockIdx.z;
   if (i2 >= f.n2) return;
   const uint64_t plane = (uint64_t)f.n1 * f.n2;
@@ -295,11 +297,13 @@ __global__ void __launch_bounds__(256) ab_signed_apply_kernel(const T* __restric
   const T v = field[k];
   if (flags[0] && !flags[1]) {
     out[k] = v;
+    if constexpr (TANGENT) out_tangent[k] = tangent[k];
     return;
   }
   auto inner = [](uint32_t i, uint32_t n) { return i < 1 ? 1u : (i > n - 2 ? n - 2 : i); };  // [1:-1] then edge padding
   const T s = smooth[(uint64_t)(inner(i0, f.n0) - s0) * plane + (uint64_t)inner(i1, f.n1) * f.n2 + inner(i2, f.n2)];
   out[k] = s > T(0.5) ? -v : v;
+  if constexpr (TANGENT) out_tangent[k] = s > T(0.5) ? -tangent[k] : tangent[k];
 }
 
 // ---- vector-field modifiers ----------------------------------------------------------------------------------------------

@@ -110,6 +110,7 @@ struct KParams {
   const void* blob[AB_MAX_BLOBS];  // (x, y, z, 0) records of T
   uint32_t blob_count[AB_MAX_BLOBS];
   const void* blob_tree[AB_MAX_BLOBS];  // device TreeRef<T> of the blob (large clouds) or nullptr: scan the blob
+  const void* dblob[AB_MAX_BLOBS];  // AB_GRAD_PARAM: tangent row of a P_FIELD blob (indexed like blob[b]), else nullptr
   // AB_GRAD_PARAM loss mode (ab_eval_grid_loss): instead of storing F and dF/dtheta the kernel accumulates
   // loss_accum[0] += sum (F - target)^2, loss_accum[1] += sum 2 (F - target) dF/dtheta   (target indexed like out)
   const T* target;
@@ -576,6 +577,21 @@ AB_DEV void load_field(const void* field, uint32_t idx, uint64_t n, Dual<Pack<T,
   load_field(field, idx, n, v);
   out = Dual<Pack<T, W>, K>(v);  // zero tangents (rejected on the host for the gradient modes anyway)
 }
+// with the tangent row of the field (AB_GRAD_PARAM: the stencil applied to d field / d theta), same index clamp; the value
+// kernels ignore it, the spatial ones never get here (the host rejects P_FIELD there)
+template <typename T, int W>
+AB_DEV void load_field(const void* field, const void*, uint32_t idx, uint64_t n, Pack<T, W>& out) {
+  load_field(field, idx, n, out);
+}
+template <typename T, int W>
+AB_DEV void load_field(const void* field, const void* dfield, uint32_t idx, uint64_t n, Dual<Pack<T, W>, 1>& out) {
+  load_field(field, idx, n, out.v);
+  load_field(dfield, idx, n, out.d[0]);
+}
+template <typename T, int W, int K>
+AB_DEV void load_field(const void* field, const void*, uint32_t idx, uint64_t n, Dual<Pack<T, W>, K>& out) {
+  load_field(field, idx, n, out);
+}
 
 // loss mode of the parameter-tangent kernel: r = F - target, sums of r^2 and 2 r dF/dtheta in double
 template <typename T, int W, int K>
@@ -965,7 +981,7 @@ __global__ void __launch_bounds__((max_threads<S, TIER>()), (big_cta<S, TIER>() 
         case D_P_SPHERE: acc = prim_sphere(p, a); break;
 #endif
 #if AB_SPEC_P_FIELD
-        case D_P_FIELD: load_field(kp.blob[sb], idx, kp.n, acc); break;
+        case D_P_FIELD: load_field(kp.blob[sb], kp.dblob[sb], idx, kp.n, acc); break;
 #endif
 #if AB_SPEC_P_CYLINDER
         case D_P_CYLINDER: acc = prim_cylinder(p, a); break;

@@ -207,8 +207,9 @@ class PinnedArray:
             pass
 
 
-_STAGED_ONLY = ("programs with grid stencils (conv_averaging / conv_edge_detection modifications) are evaluated on whole "
-                "grids only, without gradients")
+_STAGED_ONLY = ("programs with grid stencils (conv_averaging / conv_edge_detection / signed modifications) are evaluated on "
+                "grids only, without gradients in x, y, z (a stencil's output depends on the whole grid, so it has no "
+                "pointwise spatial derivative); parameter tangents (grad='param') are supported")
 
 
 def create(obj, co, *, dtype="f32", grad=None, device=0, out=None, out_grad=None, slab=None):
@@ -227,15 +228,23 @@ def create(obj, co, *, dtype="f32", grad=None, device=0, out=None, out_grad=None
     gmode, rows = _grad_mode(grad)
     spec = detect_grid(co)
     if prog.stages:
-        if spec is None or rows:
+        if spec is None or gmode == cabi.AB_GRAD_SPATIAL:
             raise NotImplementedError(_STAGED_ONLY)
         x0, x1 = (0, spec.res[0]) if slab is None else slab
         n = (x1 - x0) * spec.res[1] * spec.res[2]
         field = out if out is not None else np.empty(n, dtype=npdt)
         if field.dtype != npdt or field.size != n or not field.flags.c_contiguous:
             raise ValueError("out= must be a C-contiguous array of the evaluation dtype with N elements")
-        field[...] = _staged_torch(prog, spec, code, slab, None, device).cpu().numpy()
-        return field
+        if not rows:
+            field[...] = _staged_torch(prog, spec, code, slab, None, device).cpu().numpy()
+            return field
+        g_arr = out_grad if out_grad is not None else np.empty((rows, n), dtype=npdt)
+        if g_arr.dtype != npdt or g_arr.shape != (rows, n) or not g_arr.flags.c_contiguous:
+            raise ValueError("out_grad= must be a C-contiguous (1, N) array of the evaluation dtype")
+        f_dev, g_dev = _staged_torch(prog, spec, code, slab, None, device, param=True)
+        field[...] = f_dev.cpu().numpy()
+        g_arr[...] = g_dev.cpu().numpy()
+        return field, g_arr
     _auto_specialize(prog, dtype, grad)
     if (spec is not None and not rows and out is None and prog.n_ops == 2
             and int(prog.ops[0]["opcode"]) == oc.P_POINT_CLOUD):
@@ -299,7 +308,7 @@ def _check_stage_grid(prog, spec):
             raise ValueError("can't extend empty axis using modes other than 'constant' or 'empty'")  # np.pad
 
 
-def _staged_torch(prog, spec, code, slab, out, device, mask_gather=None):
+def _staged_torch(prog, spec, code, slab, out, device, mask_gather=None, *, param=False, out_grad=None, loss=None):
     """Programs with grid-stencil stages on the x-slab `slab` of a grid, into the torch tensor `out` (or a new one), on the
     current torch stream. Program.stage_plan says on which planes each stage is needed: in program order, the pruned
     prefix program ops[:k] is evaluated on the stage's planned range (with the fields of earlier stages bound), filtered by
@@ -312,9 +321,20 @@ def _staged_torch(prog, spec, code, slab, out, device, mask_gather=None):
     The mask of a signed stage covers every plane. Without `mask_gather` this process evaluates the stage's prefix on the
     whole axis to pack it (the cost of one whole-grid prefix evaluation per signed stage, even for a thin slab). A sharded
     evaluation passes a distributed.MaskGather: this process packs the mask of `mask_gather.planes` only, and
-    mask_gather(local_words, words_per_plane, flags) returns the whole mask (and max-reduces the two flags in place)."""
+    mask_gather(local_words, words_per_plane, flags) returns the whole mask (and max-reduces the two flags in place).
+
+    param=True carries the parameter tangent prog.dargs through the same pipeline: every stencil is linear in its field, so
+    d(stage)/d theta is the same stencil on the tangent of its input. Each prefix runs in AB_GRAD_PARAM mode into a value
+    and a tangent row, the box / edge filter runs on both rows, `signed` applies the sign pattern of the value (mask from the
+    value only) to both (ab_signed_field_slab_tangent), and each tangent row is bound to its P_FIELD op beside the field.
+    Returns (field, (1, n) tangent) into `out` / `out_grad` (a (1, >= n) tensor), or, with loss=(target, accum), runs the
+    final program through ab_eval_grid_loss (accum[0] = sum r^2, accum[1] = sum 2 r dF/dtheta over the slab) and returns
+    None."""
     import torch
     _check_stage_grid(prog, spec)
+    if param and prog.dargs is None:
+        raise ValueError("grad='param' needs Program.dargs (engine.program_tangent)")
+    gmode = cabi.AB_GRAD_PARAM if param else cabi.AB_GRAD_NONE
     dev = torch.device("cuda", device)
     stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
     tdt = torch.float32 if code == cabi.AB_F32 else torch.float64
@@ -324,38 +344,49 @@ def _staged_torch(prog, spec, code, slab, out, device, mask_gather=None):
     n0, pp = spec.res[0], spec.res[1] * spec.res[2]
     x0, x1 = (0, n0) if slab is None else (int(slab[0]), int(slab[1]))
     plan, _ = prog.stage_plan(spec.res, (x0, x1), None if mask_gather is None else mask_gather.planes)
-    fields = {}  # blob -> (device tensor, its first plane)
+    fields = {}  # blob -> (device tensor, its tangent row or None, their first plane)
     res3 = lambda m: (C.c_uint32 * 3)(m, spec.res[1], spec.res[2])
 
-    def run(p, lo, hi, dst):
-        bound = [None] * len(prog.blobs)
-        for blob, (t, p0) in fields.items():
+    def run(p, lo, hi, dst, ddst=None, target=None):
+        bound, dbound = [None] * len(prog.blobs), [None] * len(prog.blobs)
+        for blob, (t, dt, p0) in fields.items():
             if p0 <= lo and hi - p0 <= t.numel() // pp:  # the plan makes every field a program reads cover its range
                 bound[blob] = (t.data_ptr() + (lo - p0) * pp * item, (hi - lo) * pp)
-        cp = cabi.CProgram(p, device_blobs=bound)
-        codegen.ensure(p, jdt, None, is2d=_is_2d(spec))
+                if dt is not None:
+                    dbound[blob] = (dt.data_ptr() + (lo - p0) * pp * item, (hi - lo) * pp)
+        cp = cabi.CProgram(p, device_blobs=bound, device_dblobs=dbound if param else None)
+        codegen.ensure(p, jdt, "param" if param else None, is2d=_is_2d(spec))
         g = cabi.make_grid(spec.size, spec.res, (lo, hi))
-        cabi.check(lib.ab_eval_grid(cp.ref(), C.byref(g), code, cabi.AB_GRAD_NONE, C.c_void_p(dst.data_ptr()), None, 0,
+        if target is not None:
+            cabi.check(lib.ab_eval_grid_loss(cp.ref(), C.byref(g), code, C.c_void_p(target.data_ptr()),
+                                             C.c_void_p(loss[1].data_ptr()), device, stream))
+            return
+        cabi.check(lib.ab_eval_grid(cp.ref(), C.byref(g), code, gmode, C.c_void_p(dst.data_ptr()),
+                                    C.c_void_p(ddst.data_ptr()) if param else None, ddst.stride(0) if param else 0,
                                     device, stream))
+
+    def rows(m):  # value row and (param) tangent row of m samples
+        return (torch.empty(m, dtype=tdt, device=dev),
+                torch.empty((1, m), dtype=tdt, device=dev) if param else None)
 
     for st, ev, valid in plan:
         if ev is None:
             continue  # no later program reads this stage
         lo, hi = ev
         pre = prog.prefix(prog.stage_op_index(st)).pruned()  # without the subtrees an earlier stage's field replaced
-        src = torch.empty((hi - lo) * pp, dtype=tdt, device=dev)
-        run(pre, lo, hi, src)
-        if st["kind"] == 0:
-            dst = torch.empty_like(src)
-            ks = (C.c_uint32 * 3)(*st["ksize"])
-            cabi.check(lib.ab_box_filter(C.c_void_p(src.data_ptr()), res3(hi - lo), ks, st["iterations"], code,
-                                         C.c_void_p(dst.data_ptr()), device, stream))
-            fields[st["blob"]] = (dst, lo)
-        elif st["kind"] == 1:
-            dst = torch.empty_like(src)
-            cabi.check(lib.ab_edge_filter(C.c_void_p(src.data_ptr()), res3(hi - lo), code, C.c_void_p(dst.data_ptr()),
-                                          device, stream))
-            fields[st["blob"]] = (dst, lo)
+        src, dsrc = rows((hi - lo) * pp)
+        run(pre, lo, hi, src, dsrc)
+        srcs = [src] + ([dsrc] if param else [])
+        if st["kind"] in (0, 1):  # box / edge filter: linear, the tangent row takes the same stencil
+            dsts = [torch.empty_like(x) for x in srcs]
+            for a, b in zip(srcs, dsts):
+                if st["kind"] == 0:
+                    cabi.check(lib.ab_box_filter(C.c_void_p(a.data_ptr()), res3(hi - lo), (C.c_uint32 * 3)(*st["ksize"]),
+                                                 st["iterations"], code, C.c_void_p(b.data_ptr()), device, stream))
+                else:
+                    cabi.check(lib.ab_edge_filter(C.c_void_p(a.data_ptr()), res3(hi - lo), code, C.c_void_p(b.data_ptr()),
+                                                  device, stream))
+            fields[st["blob"]] = (dsts[0], dsts[1] if param else None, lo)
         else:
             words = (spec.res[2] + 31) // 32
             wpp = spec.res[1] * words  # mask words per plane
@@ -367,19 +398,37 @@ def _staged_torch(prog, spec, code, slab, out, device, mask_gather=None):
                                           C.c_void_p(flags.data_ptr()), device, stream))
             if mask_gather is not None:
                 mask = mask_gather(mask, wpp, flags)
-            dst = torch.empty((valid[1] - valid[0]) * pp, dtype=tdt, device=dev)
-            cabi.check(lib.ab_signed_field_slab(C.c_void_p(mask.data_ptr()), C.c_void_p(flags.data_ptr()),
-                                                C.c_void_p(src.data_ptr()), lo, (C.c_uint32 * 3)(*spec.res), valid[0],
-                                                valid[1], code, C.c_void_p(dst.data_ptr()), device, stream))
-            fields[st["blob"]] = (dst, valid[0])
-        del src
+            dst, ddst = rows((valid[1] - valid[0]) * pp)
+            if param:  # the value's sign pattern on both rows (the mask depends on theta only piecewise constantly)
+                cabi.check(lib.ab_signed_field_slab_tangent(
+                    C.c_void_p(mask.data_ptr()), C.c_void_p(flags.data_ptr()), C.c_void_p(src.data_ptr()),
+                    C.c_void_p(dsrc.data_ptr()), lo, (C.c_uint32 * 3)(*spec.res), valid[0], valid[1], code,
+                    C.c_void_p(dst.data_ptr()), C.c_void_p(ddst.data_ptr()), device, stream))
+            else:
+                cabi.check(lib.ab_signed_field_slab(C.c_void_p(mask.data_ptr()), C.c_void_p(flags.data_ptr()),
+                                                    C.c_void_p(src.data_ptr()), lo, (C.c_uint32 * 3)(*spec.res), valid[0],
+                                                    valid[1], code, C.c_void_p(dst.data_ptr()), device, stream))
+            fields[st["blob"]] = (dst, ddst, valid[0])
+        del src, dsrc, srcs
     n = (x1 - x0) * pp
+    # the subtrees that fed the stages are dead code now: P_FIELD overwrites their value
+    if loss is not None:
+        if loss[0].numel() != n or loss[0].dtype != tdt or not loss[0].is_contiguous():
+            raise ValueError("the target must be a contiguous tensor of the evaluation dtype with one value per slab sample")
+        run(prog.pruned(), x0, x1, None, target=loss[0])
+        return None
     if out is None:
         out = torch.empty(n, dtype=tdt, device=dev)
     elif out.numel() != n or out.dtype != tdt or not out.is_contiguous() or out.device != dev:
         raise ValueError("out= must be a contiguous CUDA tensor of the evaluation dtype with one value per slab sample")
-    run(prog.pruned(), x0, x1, out)  # the subtrees that fed the stages are dead code now: P_FIELD overwrites their value
-    return out
+    if not param:
+        run(prog.pruned(), x0, x1, out)
+        return out
+    gbuf = out_grad if out_grad is not None else torch.empty((1, (n + 7) // 8 * 8), dtype=tdt, device=dev)
+    if gbuf.dim() != 2 or gbuf.shape[1] < n or gbuf.dtype != tdt or gbuf.stride(1) != 1 or gbuf.device != dev:
+        raise ValueError("out_grad= must be a (1, >= N) CUDA tensor of the evaluation dtype with unit column stride")
+    run(prog.pruned(), x0, x1, out, gbuf)
+    return out, gbuf[:, :n]
 
 
 def create_with_gradient(obj, co, **kw):
@@ -403,6 +452,8 @@ def program_tangent(geometry, params, argnum, rel_step=1e-6):
     p0, p_lo, p_hi = (flatten(geometry(*q), fold_frames=False) for q in (params, lo, hi))
     if not (np.array_equal(p0.ops, p_lo.ops) and np.array_equal(p0.ops, p_hi.ops)):
         raise ValueError("the program structure changes with the parameter; cannot differentiate through it")
+    if not p0.stages == p_lo.stages == p_hi.stages:  # e.g. a kernel size or iteration count derived from the parameter
+        raise ValueError("a grid-stencil stage changes with the parameter; cannot differentiate through it")
     # arguments the parameter does not reach are bit-identical at theta - h and theta + h: exactly zero tangent, nothing
     # is thresholded away (a genuinely small derivative stays). The remaining tangents carry the central difference's
     # ~h^2 truncation error of the HOST-side folding (rotation matrices, frames, sin / cos of constant angles); the kernel
@@ -419,7 +470,9 @@ def jacfwd(geometry, argnums=0, *, mode="dual", dtype="f64", rel_step=1e-6, devi
         arguments as (value, d/d theta) pairs. Parameters that reach a table argument (curve-instance records,
         polyline / polygon / triangle vertices, sector tables) are not supported there.
     mode="fd": both programs at params[k] +- h evaluated in fp64 on the GPU, central difference (~1e-9 relative);
-        works for every op."""
+        works for every op.
+    Trees with grid-stencil stages take both modes on grids: in dual mode the tangent goes through the same stencils
+    (_staged_torch)."""
 
     def grad_map_dual(co, *params):
         prog = program_tangent(geometry, params, argnums, rel_step)
@@ -468,16 +521,22 @@ def value_and_grad(geometry, spec, target, *, dtype="f32", device=0, post=None, 
         grads, loss = [], None
         for k in range(len(params)):
             prog = program_tangent(geometry, params, k)
+            if specialized and prog.stages:
+                raise NotImplementedError("specialized=True does not cover trees with grid stencils (their prefix programs "
+                                          "run on the general or program-compiled kernels); call without it")
             if specialized:  # one compilation per op set (cached); later steps of the optimisation loop reuse it
                 specialize(prog, dtype=dtype, grad="param")
             if post is None:
                 # fused: the kernel reduces sum r^2 and sum 2 r dF/dtheta_k itself (ab_eval_grid_loss), nothing is stored
-                cp = cabi.CProgram(prog)
-                codegen.ensure(prog, "f32" if code == cabi.AB_F32 else "f64", "param", is2d=_is_2d(spec))
-                g = cabi.make_grid(spec.size, spec.res)
-                stream = torch.cuda.current_stream(dev).cuda_stream
-                cabi.check(cabi.lib().ab_eval_grid_loss(cp.ref(), C.byref(g), code, tgt.data_ptr(), accum.data_ptr(), device,
-                                                        C.c_void_p(stream)))
+                if prog.stages:  # the staged pipeline, with the reduction in the final program's kernel
+                    _staged_torch(prog, spec, code, None, None, device, param=True, loss=(tgt, accum))
+                else:
+                    cp = cabi.CProgram(prog)
+                    codegen.ensure(prog, "f32" if code == cabi.AB_F32 else "f64", "param", is2d=_is_2d(spec))
+                    g = cabi.make_grid(spec.size, spec.res)
+                    stream = torch.cuda.current_stream(dev).cuda_stream
+                    cabi.check(cabi.lib().ab_eval_grid_loss(cp.ref(), C.byref(g), code, tgt.data_ptr(), accum.data_ptr(),
+                                                            device, C.c_void_p(stream)))
                 both = accum.cpu()
                 if loss is None:
                     loss = float(both[0])
@@ -502,14 +561,17 @@ def create_torch(obj, spec: GridSpec, *, dtype="f32", grad=None, device=0, slab=
                  mask_gather=None):
     """Grid evaluation into torch CUDA tensors on the current torch stream (no host copy). Returns field
     (and gradient (3,N) view of a row-padded buffer). Programs with grid-stencil stages evaluate their stages on the
-    slab plus the halo they need (_staged_torch, where `mask_gather` is described); they take no gradient."""
+    slab plus the halo they need (_staged_torch, where `mask_gather` is described); they take grad='param' (the tangent
+    goes through the same stencils) but no spatial gradient."""
     import torch
     prog = _as_program(obj)
     code, npdt = _dtype(dtype)
     if prog.stages:
-        if grad not in (None, False, "none"):
+        gmode, _ = _grad_mode(grad)
+        if gmode == cabi.AB_GRAD_SPATIAL:
             raise NotImplementedError(_STAGED_ONLY)
-        return _staged_torch(prog, spec, code, slab, out, device, mask_gather)
+        return _staged_torch(prog, spec, code, slab, out, device, mask_gather, param=gmode == cabi.AB_GRAD_PARAM,
+                             out_grad=out_grad)
     _auto_specialize(prog, dtype, grad)
     codegen.ensure(prog, "f32" if code == cabi.AB_F32 else "f64", grad, is2d=_is_2d(spec))
     tdt = torch.float32 if code == cabi.AB_F32 else torch.float64

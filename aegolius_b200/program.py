@@ -78,6 +78,7 @@ class Program:
         ops = np.concatenate([self.ops[:op_index], np.array([(oc.END, 0, 0, 0)], dtype=OP_DTYPE)])
         pre = Program(ops, self.args, self.blobs, self.n_pslots, self.n_vslots,
                       [st for st in self.stages if self.stage_op_index(st) < op_index])
+        pre.dargs = self.dargs  # the argument pool is shared and its offsets absolute: the same tangent applies
         return pre
 
     def stage_plan(self, res, slab=None, mask_planes=None):
@@ -205,7 +206,9 @@ class Program:
         if keep.all():
             return self
         out = np.concatenate([ops[keep], self.ops[-1:]])
-        return Program(out, self.args, self.blobs, self.n_pslots, self.n_vslots, list(self.stages))
+        kept = Program(out, self.args, self.blobs, self.n_pslots, self.n_vslots, list(self.stages))
+        kept.dargs = self.dargs
+        return kept
 
     @classmethod
     def from_arrays(cls, d, prefix="prog_"):

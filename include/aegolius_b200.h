@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define AB_VERSION 101 /* 0.1.1 */
+#define AB_VERSION 102 /* 0.1.2 */
 
 typedef enum ab_status {
   AB_OK = 0,
@@ -42,7 +42,8 @@ typedef enum ab_grad_mode {
   AB_GRAD_SPATIAL = 1, /* d field / d(x,y,z): analytic counterpart of from_sdf (vector_functions.py:130-139) */
   AB_GRAD_PARAM = 2    /* d field / d theta for one scalar parameter: replaces jacfwd(geometry, argnums=k),
                           Code/examples/autodiff/gradient_map_3D.py:84. ab_program.dargs holds d args / d theta; every
-                          argument is read as a dual number and the tangent is propagated op by op. Limits: at most
+                          argument is read as a dual number and the tangent is propagated op by op (P_FIELD reads its
+                          tangent from ab_program.dblobs). Limits: at most
                           AB_MAX_ARGS/2 arguments; table arguments (instance / vertex / sector tables, per-quadrant
                           radii, norm order) must have zero tangent (AB_EUNSUPPORTED_OP otherwise). */
 } ab_grad_mode;
@@ -131,8 +132,10 @@ typedef enum ab_opcode {
   AB_OP_P_POINT_CLOUD = 114, /* a = dim (2|3), b = blob index: nearest-point distance (sdf_3D.py:283-286) */
   AB_OP_P_FIELD = 115,       /* b = blob index of a DEVICE field (blob.dim = 1, one value of the evaluation dtype per point
                                 of the call, indexed like `out`): value = field[point]. Carries the output of a grid
-                                stencil (conv_averaging / conv_edge_detection as a modification,
-                                modifications.py:1586-1637) back into the op list; no derivative passes through it */
+                                stencil (conv_averaging / conv_edge_detection / signed as a modification,
+                                modifications.py:220-275, 1586-1637) back into the op list. Under AB_GRAD_PARAM the
+                                tangent is ab_program.dblobs[b][point] (the stencil applied to the tangent of its input);
+                                no spatial derivative passes through it */
   /* --- 2D primitives (sdf_2D.py), evaluated on (x,y) --- */
   AB_OP_P_CIRCLE = 128, AB_OP_P_NEU_CIRCLE = 129, AB_OP_P_BOX2D = 130, AB_OP_P_SEGMENT2D = 131,
   AB_OP_P_RBOX2D = 132, AB_OP_P_TRIANGLE2D = 133, AB_OP_P_ARC = 134, AB_OP_P_SECTOR = 135,
@@ -161,6 +164,9 @@ typedef struct ab_program {
   uint32_t n_blobs;
   uint32_t n_pslots;   /* P-slots used (<= AB_MAX_PSLOTS) */
   uint32_t n_vslots;   /* V-slots used (<= AB_MAX_VSLOTS) */
+  const ab_blob* dblobs; /* NULL, or n_blobs entries: entry b is the DEVICE tangent row d field_b / d theta of a P_FIELD blob
+                            (dim = 1, indexed and advanced exactly like blob b). AB_GRAD_PARAM needs one for every P_FIELD
+                            blob the program reads; other entries and other modes ignore it */
 } ab_program;
 
 /* Regular grid exactly as generate_grid builds it (helper_functions.py:23-93): per axis
@@ -286,6 +292,13 @@ int ab_signed_mask(const void* field_dev, const uint32_t res[3], double threshol
 int ab_signed_field_slab(const uint32_t* mask_dev, const int* flags_dev, const void* field_dev, uint32_t field_plane0,
                          const uint32_t res[3], uint32_t x0, uint32_t x1, int dtype, void* out_dev, int device,
                          void* stream);
+/* ab_signed_field_slab on a field and its parameter tangent at once (tangent_dev laid out like field_dev, out_tangent_dev
+ * like out_dev): one interior and smoothing, then out = +-field and out_tangent = +-tangent with the same sign per sample.
+ * The mask and flags come from the field's values only (the boundary mask is piecewise constant in the parameter); when the
+ * field had a negative sample and no NaN both pass through unchanged. out_dev bit-identical to ab_signed_field_slab. */
+int ab_signed_field_slab_tangent(const uint32_t* mask_dev, const int* flags_dev, const void* field_dev,
+                                 const void* tangent_dev, uint32_t field_plane0, const uint32_t res[3], uint32_t x0,
+                                 uint32_t x1, int dtype, void* out_dev, void* out_tangent_dev, int device, void* stream);
 
 /* Vector-field modifiers (vector_modification_functions.py:14-172; methods modifications.py:1712-1971). */
 #define AB_MAX_VEC_OPS 32

@@ -59,6 +59,20 @@ def items():
         for dt in ("f32", "f64"):
             for g in (None, "spatial"):
                 out.append((prog, dt, g, False))
+    # parameter tangents through grid-stencil stages (tests/test_gpu_stage_tangents.py, tools/stage_tangent_probe.py): the
+    # pruned prefixes and the final program of each tangent program, in parameter mode and in value mode (differences)
+    sys.path.insert(0, os.path.join(ROOT, "tools"))
+    import stage_tangent_probe
+    import test_gpu_stage_tangents
+    from aegolius_b200.engine import program_tangent
+    staged = [(program_tangent(builder, p, k), len(res) == 2)
+              for builder, p, _, res, _ in test_gpu_stage_tangents.BUILDERS.values() for k in range(len(p))]
+    staged += [(prog, False) for _, prog, _ in stage_tangent_probe.programs()]
+    for prog, is2d in staged:
+        for q in [prog.pruned()] + [prog.prefix(prog.stage_op_index(st)).pruned() for st in prog.stages]:
+            for dt in ("f32", "f64"):
+                for g in (None, "param"):
+                    out.append((q, dt, g, is2d))
     return out
 
 
